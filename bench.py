@@ -2,6 +2,7 @@
 """bench.py — the Decoder hot path on B200: log lines/s and GB/s parsed, with roofline + CPU baseline.
 
     python bench.py --gpus N --steps K --warmup W [--format rfc5424|ltsv|gelf|rfc3164|mixed] [--lines L] [--impl reference]
+                    [--dump-outputs DIR]
 
 A "step" is one pass of the parse kernel over one synthetic batch that is already resident in HBM
 (BASELINE.json configs[1]: 10 M RFC5424 lines, mean 180 B, per GPU).  `e2e` is the same metric through
@@ -31,6 +32,9 @@ RFC3164_YEAR = 2026  # the year timestamps without one belong to: fixed, so that
 GEN_MEAN = {"rfc5424": 169.2, "ltsv": 420.0, "gelf": 466.0, "rfc3164": 140.0}
 TARGET_MEAN = {"rfc5424": 180, "ltsv": 420, "gelf": 512, "rfc3164": 127}
 DEFAULT_LINES = {"rfc5424": 10_000_000, "ltsv": 4_000_000, "gelf": 3_500_000, "rfc3164": 10_000_000}  # int32 offsets cap a batch at 2 GiB
+DUMP_BYTES = 60 << 20  # --dump-outputs writes at most this much array data (stays under 64 MB with the .npy headers)
+DUMP_SEED = 0
+DUMP_BLOCK = 64  # --dump-outputs samples blocks of this many consecutive lines
 
 
 def env_int(name: str, default: int) -> int:
@@ -156,6 +160,41 @@ def oracle_config(pyoracle, fmt_name: str, typed: bool):
     return None
 
 
+def dump_outputs(decoded: dict, out_dir: str, budget: int) -> None:
+    """--dump-outputs: the Records of decoded batches ({file name prefix: (BatchDecoder, BatchResult, bytes, offsets)}) as
+    the product's host library materialises them for a caller, in the canonical dump format of oracle/oracle.cpp (every
+    field, ts as its bits).  The raw result arrays are not written: the kernels fill their side tables in a different order
+    from run to run.  For each prefix, in `out_dir`:
+        <prefix>line.npy            float64 [k]    the line numbers dumped, ascending
+        <prefix>record_offsets.npy  float64 [k+1]  record i is record_bytes[offsets[i]:offsets[i+1]]
+        <prefix>record_bytes.npy    float32        the dump text, one byte per element
+    The lines are blocks of DUMP_BLOCK consecutive lines, taken in a seeded order until the prefix's share of `budget`
+    (bytes of array data) is used."""
+    import numpy as np
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    share = budget // max(len(decoded), 1) - 8
+    for prefix, (dec, res, data, offsets) in decoded.items():
+        blocks, used = [], 0
+        for lo in np.random.default_rng(DUMP_SEED).permutation(-(-res.n // DUMP_BLOCK)) * DUMP_BLOCK:
+            lo = int(lo)
+            hi = min(res.n, lo + DUMP_BLOCK)
+            text, offs = dec.dump(res, data, offsets, nthreads=1, lo=lo, hi=hi)
+            cost = 4 * len(text) + 16 * (hi - lo)  # float32 per byte, float64 line number and offset per line
+            if used + cost > share:
+                break
+            blocks.append((lo, hi, text, offs))
+            used += cost
+        blocks.sort(key=lambda b: b[0])
+        lines = [np.arange(lo, hi) for lo, hi, _, _ in blocks]
+        lengths = [np.diff(offs) for _, _, _, offs in blocks]
+        rec_offs = np.zeros(sum(len(x) for x in lines) + 1)
+        np.cumsum(np.concatenate(lengths) if lengths else [], out=rec_offs[1:])
+        np.save(out / f"{prefix}line.npy", np.concatenate(lines).astype(np.float64) if lines else np.zeros(0))
+        np.save(out / f"{prefix}record_offsets.npy", rec_offs)
+        np.save(out / f"{prefix}record_bytes.npy", np.frombuffer(b"".join(b[2] for b in blocks), np.uint8).astype(np.float32))
+
+
 def run_reference(args) -> None:
     """CPU arm: the restated reference decoders (oracle/) on the host cores, same workload shape."""
     rank = env_int("RANK", 0)
@@ -269,6 +308,10 @@ def run_mixed(args) -> None:
     wall = reduce(time.perf_counter() - t0, torch.distributed.ReduceOp.MAX if dist else None)
     clocks = sampler.stop() if rank == 0 else None
     launches = sum(d[1].kernel_launches() for d in decs) - launches0
+    if args.dump_outputs:  # before the e2e decodes below overwrite the results of the last timed step
+        rank_prefix = f"rank{rank}." if world > 1 else ""
+        dump_outputs({f"{rank_prefix}{k}.{f}.": (dec, dec.download(), hb, ho) for k, (f, dec, hb, ho, *_) in enumerate(decs)},
+                     args.dump_outputs, DUMP_BYTES // world)
     per_gpu = tot_lines / (wall / args.steps)
     total_lines = reduce(float(tot_lines), torch.distributed.ReduceOp.SUM if dist else None)
     total_bytes = reduce(float(tot_bytes), torch.distributed.ReduceOp.SUM if dist else None)
@@ -352,7 +395,14 @@ def main() -> None:
     ap.add_argument("--split", action="store_true", help="also time fg_split_decode (device-side framing + UTF-8 validation, N1)")
     ap.add_argument("--ltsv-typed", action="store_true", help="LTSV with the 4-entry typed schema + suffixes (C4, second run)")
     ap.add_argument("--encode", action="store_true", help="also time fg_decode_encode_gelf (decode + GELF encode fused on the device, N2)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the Records of the last step to DIR/<name>.npy (a seeded sample of "
+                         "lines, 60 MiB at most; see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU decoder's outputs; --impl reference has none")
     if args.format == "mixed":
         if args.lines <= 0:
             args.lines = 12_500_000
@@ -448,7 +498,7 @@ def main() -> None:
 
     # the dominant kernel alone (RFC5424: parse5424_kernel, without post5424_kernel), CUDA events around it, single steps
     dom = []
-    for _ in range(max(args.steps, 10)):
+    for _ in range(args.steps):
         dec.parse_resident()
         dom.append(dec.last_dominant_kernel_ms())
     dom_ms = max_over_ranks(sum(dom) / len(dom))
@@ -462,6 +512,8 @@ def main() -> None:
     else:
         b_write = n * (12 + 8 * 4) + n_entries * 17 + (int(res.raw.arena_bytes) if fmt == 3 else 0)
     d2h_bytes = b_write
+    if args.dump_outputs:  # the last timed step's results, before the e2e decodes below overwrite them
+        dump_outputs({f"rank{rank}." if world > 1 else "": (dec, res, h_bytes, h_offs)}, args.dump_outputs, DUMP_BYTES // world)
 
     # ---- end to end through the C ABI with host buffers -----------------------------------------
     dec.decode(h_bytes, h_offs)  # warm-up
