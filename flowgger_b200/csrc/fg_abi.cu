@@ -87,10 +87,59 @@ struct ErrorTableInit {
 constexpr size_t kPad = 256;            // slack after the device byte buffer (16-byte bulk-copy granules)
 constexpr size_t kBounceBytes = 32u << 20;  // pinned bounce buffers for pageable caller memory
 constexpr size_t kL2FlushBytes = 256u << 20;
-constexpr int kCnt = 8;                 // u32 counters snapshotted per chunk (fg::K5_* + the bad-offsets flag)
-constexpr int kBadFlag = 6;             // d_k[kBadFlag]: set by check_offsets_kernel
+constexpr int kRedo = 1;  // drain(): tables were regrown and the attempt must be enqueued again (FG_E_* codes are negative)
+const char* const kBadOffsets = "offsets must be non-decreasing and within max_batch_bytes";
+
+// A device array, its pinned host mirror and their capacity in elements of `width` bytes.  alloc() rounds the
+// capacity up to a multiple of `round` and allocates `pad` bytes more on both sides.
+struct Mirror {
+    const size_t width, round, pad;
+    uint8_t* d = nullptr;
+    uint8_t* h = nullptr;
+    size_t cap = 0;
+
+    explicit Mirror(size_t width_, size_t round_ = 1, size_t pad_ = 0) : width(width_), round(round_), pad(pad_) {}
+    Mirror(const Mirror&) = delete;
+    Mirror& operator=(const Mirror&) = delete;
+    ~Mirror() { release(); }
+
+    void release() {
+        if (d) cudaFree(d);
+        if (h) cudaFreeHost(h);
+        d = h = nullptr;
+        cap = 0;
+    }
+    cudaError_t alloc(size_t n) {
+        release();
+        n = (n + round - 1) / round * round;
+        cudaError_t e = cudaMalloc(&d, n * width + pad);
+        if (e == cudaSuccess) e = cudaHostAlloc(&h, n * width + pad, cudaHostAllocDefault);
+        if (e == cudaSuccess) cap = n;
+        return e;
+    }
+    // elements [from, to) back to the host mirror
+    cudaError_t d2h(size_t from, size_t to, cudaStream_t s) const {
+        if (to <= from) return cudaSuccess;
+        return cudaMemcpyAsync(h + from * width, d + from * width, (to - from) * width, cudaMemcpyDeviceToHost, s);
+    }
+    template <class T>
+    T* dev() const { return (T*)d; }
+    template <class T>
+    T* host() const { return (T*)h; }
+};
+
+// One result table of a format: the counter (fg::K5_*) that bounds it, the mirrors that hold it (one per column, all
+// with the same capacity) and the capacity a format allocates when it finds the table empty.
+struct Table {
+    int slot;
+    std::vector<Mirror*> cols;
+    size_t first;
+    bool grow_to_first;  // also grown to `first` when another format left it smaller
+};
 
 }  // namespace
+
+static_assert(sizeof(fg_wide_row) == sizeof(fg::WideRow), "wide rows are copied back byte for byte");
 
 struct fg_ctx {
     int device = 0;
@@ -98,53 +147,34 @@ struct fg_ctx {
     int max_lines = 0;
     int chunk_lines = 0;
     cudaStream_t s_h2d = nullptr, s_comp = nullptr, s_d2h = nullptr;
-    // device: input
+    // device: input; the host side receives the line offsets fg_split_decode finds
     uint8_t* d_bytes = nullptr;
-    int32_t* d_offsets = nullptr;
-    uint32_t* d_k = nullptr;  // counter block (fg::K5_* ; [kBadFlag] = offsets check)
+    Mirror offsets{sizeof(int32_t)};
+    uint32_t* d_k = nullptr;  // counter block (fg::K5_*)
     uint8_t* d_flush = nullptr;
-    // LTSV / GELF: columnar rows (9 columns sized for max_lines) + 17-byte side-table rows + scratch.
-    // The side-table arrays also hold the rows of the RFC5424 wide lines.
-    uint8_t* d_rows = nullptr;
-    uint8_t* h_rows = nullptr;
-    int2* d_entry_name = nullptr;
-    unsigned long long* d_entry_val = nullptr;
-    uint8_t* d_entry_meta = nullptr;
-    fg_span* h_entry_name = nullptr;
-    uint64_t* h_entry_val = nullptr;
-    uint8_t* h_entry_meta = nullptr;
-    size_t entry_cap = 0;
+    // LTSV / GELF / RFC3164: columnar rows (9 columns sized for max_lines)
+    Mirror rows{1};
+    // 17-byte side-table rows (LTSV / GELF, RFC5424 wide lines) + LTSV / GELF scratch
+    Mirror entry_name{sizeof(fg_span), 256}, entry_val{sizeof(uint64_t), 256}, entry_meta{1, 256};
     int2* d_tmp_name = nullptr;  // provisional side-table rows, indexed by byte offset / scratch_div
     unsigned long long* d_tmp_val = nullptr;
     uint8_t* d_tmp_meta = nullptr;
     size_t tmp_cap = 0;
     // RFC5424: compact rows, 8-byte entries, work lists, arena, wide rows
-    uint4* d_rows5 = nullptr;
-    fg_row5424* h_rows5 = nullptr;
-    unsigned long long* d_e8 = nullptr;
-    uint64_t* h_e8 = nullptr;
-    size_t e8_cap = 0;
+    Mirror rows5{sizeof(fg_row5424)};
+    Mirror e8{8, 256};
     uint32_t* d_esc_list = nullptr;
-    uint32_t* d_wide_list = nullptr;
-    uint8_t* d_arena = nullptr;
-    uint8_t* h_arena = nullptr;
-    size_t arena_cap = 0;
-    fg::WideRow* d_wide = nullptr;
-    fg_wide_row* h_wide = nullptr;
-    size_t wide_cap = 0;
+    uint32_t* d_wide_list = nullptr;  // RFC5424 wide lines, GELF slow lines
+    Mirror arena{1, 256};
+    Mirror wide{sizeof(fg_wide_row)};
+    std::vector<Table> tables[4];  // by fg_format (list_tables)
     // fused GELF encoder (fg_decode_encode_gelf)
     uint32_t* d_enc_lens = nullptr;
     uint32_t* d_enc_rel = nullptr;
-    unsigned long long* d_enc_base = nullptr;  // [chunks + 1] running output size
-    unsigned long long* h_enc_base = nullptr;
-    int enc_base_cap = 0;
-    uint8_t* d_enc_out = nullptr;
-    uint8_t* h_enc_out = nullptr;
-    size_t enc_out_cap = 0;
-    long long* d_enc_offsets = nullptr;
-    int64_t* h_enc_offsets = nullptr;
-    uint8_t* d_enc_status = nullptr;
-    uint8_t* h_enc_status = nullptr;
+    Mirror enc_base{sizeof(unsigned long long)};  // [chunks + 1] running output size
+    Mirror enc_out{1, 4096, 16};
+    Mirror enc_offsets{sizeof(int64_t)};
+    Mirror enc_status{1};
     void* d_scan_temp = nullptr;
     size_t scan_temp_bytes = 0;
     uint8_t* d_static_blob = nullptr;  // fixed GELF keys + output.gelf_extra, sorted
@@ -157,14 +187,12 @@ struct fg_ctx {
     uint32_t* d_seg = nullptr;
     int32_t* d_n_lines = nullptr;
     uint8_t* d_invalid = nullptr;
-    int32_t* h_offsets = nullptr;
     int32_t* h_n_lines = nullptr;
     float last_split_ms = 0.f;
     cudaEvent_t ev_s0 = nullptr, ev_s1 = nullptr;
     cudaStream_t s_parse = nullptr;
     std::vector<cudaEvent_t> ev_split;
-    int32_t* d_cum = nullptr;
-    int32_t* h_cum = nullptr;
+    Mirror cum{sizeof(int32_t)};
     // RFC3164: the year `now_utc().year()` stands for (0: read the clock at every call) and the zone database
     int r3164_year = 0;
     int call_year = 1970;  // the year of the call in progress (current_year())
@@ -176,7 +204,7 @@ struct fg_ctx {
     uint8_t* d_ltsv_blob = nullptr;
     fg::LtsvDeviceConfig ltsv{};
     // pinned host
-    uint32_t* h_counts = nullptr;  // per-chunk snapshots of the counter block (kCnt words each)
+    uint32_t* h_counts = nullptr;  // per-step snapshots of the counter block (fg::K5_COUNT words each)
     int h_counts_cap = 0;
     uint8_t* h_bounce[2] = {nullptr, nullptr};
     cudaEvent_t bounce_ev[2] = {nullptr, nullptr};
@@ -188,7 +216,7 @@ struct fg_ctx {
     int res_n = 0;
     size_t res_bytes = 0;
     int res_fmt = -1;
-    uint32_t res_tot[kCnt] = {};
+    uint32_t res_tot[fg::K5_COUNT] = {};
     std::string last_error;
     int64_t launches = 0;
     int max_tile = 0;   // LTSV / GELF staging tile limit
@@ -234,74 +262,49 @@ void hfree(T*& p) {
     p = nullptr;
 }
 
-// 17-byte side-table rows (LTSV / GELF, RFC5424 wide lines)
-int alloc_entries(fg_ctx* c, size_t cap) {
-    dfree(c->d_entry_name); dfree(c->d_entry_val); dfree(c->d_entry_meta);
-    hfree(c->h_entry_name); hfree(c->h_entry_val); hfree(c->h_entry_meta);
-    c->entry_cap = 0;
-    cap = (cap + 255) & ~(size_t)255;
-    FG_CUDA(c, cudaMalloc(&c->d_entry_name, cap * sizeof(int2)));
-    FG_CUDA(c, cudaMalloc(&c->d_entry_val, cap * sizeof(unsigned long long)));
-    FG_CUDA(c, cudaMalloc(&c->d_entry_meta, cap));
-    FG_CUDA(c, cudaHostAlloc(&c->h_entry_name, cap * sizeof(fg_span), cudaHostAllocDefault));
-    FG_CUDA(c, cudaHostAlloc(&c->h_entry_val, cap * sizeof(uint64_t), cudaHostAllocDefault));
-    FG_CUDA(c, cudaHostAlloc(&c->h_entry_meta, cap, cudaHostAllocDefault));
-    c->entry_cap = cap;
-    return FG_OK;
+uint32_t cap32(const Mirror& m) { return (uint32_t)std::min<size_t>(m.cap, 0xFFFFFFFFu); }
+
+// The result tables of every format; capacities are in elements.  RFC3164 fills no side-table rows, but its results
+// still point at an (empty) entries table.
+void list_tables(fg_ctx* c) {
+    const size_t mb = c->max_bytes;
+    const std::vector<Mirror*> entries = {&c->entry_name, &c->entry_val, &c->entry_meta};
+    c->tables[FG_FMT_RFC5424] = {{fg::K5_ENTRIES, {&c->e8}, std::max<size_t>(mb / 24, 4096), false},
+                                 {fg::K5_ARENA, {&c->arena}, std::max<size_t>(mb / 64, 64 << 10), false},
+                                 {fg::K5_WIDE_ROWS, {&c->wide}, 1024, false},
+                                 {fg::K5_WIDE_ENTRIES, entries, 4096, false}};
+    c->tables[FG_FMT_LTSV] = {{fg::K5_ENTRIES, entries, std::max<size_t>(mb / 24, 4096), true}};
+    c->tables[FG_FMT_GELF] = c->tables[FG_FMT_LTSV];
+    c->tables[FG_FMT_RFC3164] = {{fg::K5_ARENA, {&c->arena}, std::max<size_t>(mb / 32, 64 << 10), false},
+                                 {fg::K5_ENTRIES, entries, 256, false}};
 }
-int alloc_e8(fg_ctx* c, size_t cap) {
-    dfree(c->d_e8); hfree(c->h_e8);
-    c->e8_cap = 0;
-    cap = (cap + 255) & ~(size_t)255;
-    FG_CUDA(c, cudaMalloc(&c->d_e8, cap * 8));
-    FG_CUDA(c, cudaHostAlloc(&c->h_e8, cap * 8, cudaHostAllocDefault));
-    c->e8_cap = cap;
-    return FG_OK;
-}
-int alloc_arena(fg_ctx* c, size_t cap) {
-    dfree(c->d_arena); hfree(c->h_arena);
-    c->arena_cap = 0;
-    cap = (cap + 255) & ~(size_t)255;
-    FG_CUDA(c, cudaMalloc(&c->d_arena, cap));
-    FG_CUDA(c, cudaHostAlloc(&c->h_arena, cap, cudaHostAllocDefault));
-    c->arena_cap = cap;
-    return FG_OK;
-}
-int alloc_wide(fg_ctx* c, size_t cap) {
-    dfree(c->d_wide); hfree(c->h_wide);
-    c->wide_cap = 0;
-    FG_CUDA(c, cudaMalloc(&c->d_wide, cap * sizeof(fg::WideRow)));
-    FG_CUDA(c, cudaHostAlloc(&c->h_wide, cap * sizeof(fg_wide_row), cudaHostAllocDefault));
-    c->wide_cap = cap;
-    return FG_OK;
-}
+
+// Host arrays packed into one device allocation: every piece at a 16-byte aligned offset, 16 zero bytes after the last.
+struct Blob {
+    std::vector<uint8_t> bytes;
+    template <class V>
+    size_t put(const V& v) {  // a std::vector or std::string; returns its offset
+        const size_t at = bytes.size();
+        const uint8_t* p = (const uint8_t*)v.data();
+        bytes.insert(bytes.end(), p, p + v.size() * sizeof(v[0]));
+        bytes.resize((bytes.size() + 15) & ~(size_t)15, 0);
+        return at;
+    }
+    cudaError_t upload(uint8_t*& d) {  // replaces d
+        bytes.resize(bytes.size() + 16, 0);
+        dfree(d);
+        const cudaError_t e = cudaMalloc(&d, bytes.size());
+        return e != cudaSuccess ? e : cudaMemcpy(d, bytes.data(), bytes.size(), cudaMemcpyHostToDevice);
+    }
+};
 
 // packed zone table -> one device blob (fg::TzDeviceTable points into it)
 int upload_tz(fg_ctx* c) {
     const fg::TzHostTable& H = c->tz_host;
-    dfree(c->d_tz_blob);
-    size_t o = 0;
-    auto place = [&](size_t bytes) {
-        const size_t at = o;
-        o += (bytes + 15) & ~(size_t)15;
-        return at;
-    };
-    const size_t o_hash = place(H.hash.size() * 8), o_key = place(H.key.size() * 8), o_zone = place(H.zone.size() * 4),
-                 o_noff = place(H.name_off.size() * 4), o_first = place(H.first.size() * 4), o_off = place(H.off.size() * 4),
-                 o_names = place(H.names.size());
-    std::vector<uint8_t> blob(o + 16, 0);
-    auto put = [&](size_t at, const void* src, size_t bytes) {
-        if (bytes) memcpy(blob.data() + at, src, bytes);
-    };
-    put(o_hash, H.hash.data(), H.hash.size() * 8);
-    put(o_key, H.key.data(), H.key.size() * 8);
-    put(o_zone, H.zone.data(), H.zone.size() * 4);
-    put(o_noff, H.name_off.data(), H.name_off.size() * 4);
-    put(o_first, H.first.data(), H.first.size() * 4);
-    put(o_off, H.off.data(), H.off.size() * 4);
-    put(o_names, H.names.data(), H.names.size());
-    FG_CUDA(c, cudaMalloc(&c->d_tz_blob, blob.size()));
-    FG_CUDA(c, cudaMemcpy(c->d_tz_blob, blob.data(), blob.size(), cudaMemcpyHostToDevice));
+    Blob b;
+    const size_t o_hash = b.put(H.hash), o_key = b.put(H.key), o_zone = b.put(H.zone), o_noff = b.put(H.name_off),
+                 o_first = b.put(H.first), o_off = b.put(H.off), o_names = b.put(H.names);
+    FG_CUDA(c, b.upload(c->d_tz_blob));
     fg::TzDeviceTable& T = c->tz_dev;
     T = H.view();
     T.hash = (const unsigned long long*)(c->d_tz_blob + o_hash);
@@ -325,33 +328,20 @@ int current_year(const fg_ctx* c) {
 
 // Format-specific buffers are allocated on first use of the format.
 int ensure_format(fg_ctx* c, int fmt) {
-    if (fmt == FG_FMT_RFC5424) {
-        if (!c->d_rows5) {
-            FG_CUDA(c, cudaMalloc(&c->d_rows5, (size_t)c->max_lines * 32));
-            FG_CUDA(c, cudaHostAlloc(&c->h_rows5, (size_t)c->max_lines * 32, cudaHostAllocDefault));
-            FG_CUDA(c, cudaMalloc(&c->d_esc_list, (size_t)c->max_lines * 4));
-            FG_CUDA(c, cudaMalloc(&c->d_wide_list, (size_t)c->max_lines * 4));
-        }
-        if (!c->e8_cap)
-            if (int rc = alloc_e8(c, std::max<size_t>(c->max_bytes / 24, 4096))) return rc;
-        if (!c->arena_cap)
-            if (int rc = alloc_arena(c, std::max<size_t>(c->max_bytes / 64, 64 << 10))) return rc;
-        if (!c->wide_cap)
-            if (int rc = alloc_wide(c, 1024)) return rc;
-        if (!c->entry_cap)
-            if (int rc = alloc_entries(c, 4096)) return rc;
-        return FG_OK;
+    if (fmt == FG_FMT_RFC5424 && !c->rows5.cap) {
+        FG_CUDA(c, c->rows5.alloc(c->max_lines));
+        FG_CUDA(c, cudaMalloc(&c->d_esc_list, (size_t)c->max_lines * 4));
     }
-    if (!c->d_rows) {
-        const size_t rows_bytes = col_off(c, C_COUNT);
-        FG_CUDA(c, cudaMalloc(&c->d_rows, rows_bytes));
-        FG_CUDA(c, cudaHostAlloc(&c->h_rows, rows_bytes, cudaHostAllocDefault));
+    if (fmt != FG_FMT_RFC5424 && !c->rows.cap) FG_CUDA(c, c->rows.alloc(col_off(c, C_COUNT)));
+    if ((fmt == FG_FMT_RFC5424 || fmt == FG_FMT_GELF) && !c->d_wide_list)
+        FG_CUDA(c, cudaMalloc(&c->d_wide_list, (size_t)c->max_lines * 4));
+    for (const Table& t : c->tables[fmt]) {
+        const size_t cap = t.cols[0]->cap;
+        if (t.grow_to_first ? cap < t.first : cap == 0)
+            for (Mirror* m : t.cols) FG_CUDA(c, m->alloc(t.first));
     }
-    if (fmt == FG_FMT_RFC3164) {  // no side table; re-joined messages go to the arena; zone names need the database
-        if (!c->arena_cap)
-            if (int rc = alloc_arena(c, std::max<size_t>(c->max_bytes / 32, 64 << 10))) return rc;
-        if (!c->entry_cap)
-            if (int rc = alloc_entries(c, 256)) return rc;
+    if (fmt == FG_FMT_RFC5424) return FG_OK;
+    if (fmt == FG_FMT_RFC3164) {  // zone names need the database
         if (!c->tz_host.loaded) {
             std::string err;
             if (!fg::tz_load_dir(c->tzdir.empty() ? nullptr : c->tzdir.c_str(), c->tz_host, err)) return fail(c, FG_E_ARG, err.c_str());
@@ -360,10 +350,6 @@ int ensure_format(fg_ctx* c, int fmt) {
             if (int rc = upload_tz(c)) return rc;
         return FG_OK;
     }
-    if (fmt == FG_FMT_GELF && !c->d_wide_list) FG_CUDA(c, cudaMalloc(&c->d_wide_list, (size_t)c->max_lines * 4));  // slow list
-    const size_t want = std::max<size_t>(c->max_bytes / 24, 4096);
-    if (c->entry_cap < want)
-        if (int rc = alloc_entries(c, want)) return rc;
     // Scratch table for provisional side-table rows, indexed by byte offset (see Format<>::scratch_index):
     // a row needs >= 3 input bytes in GELF, >= 1 byte + its TAB in LTSV.
     const size_t need = (fmt == FG_FMT_LTSV ? c->max_bytes / 2 + (size_t)c->max_lines : c->max_bytes / 3) + 64;
@@ -394,27 +380,18 @@ int pick_tile(const fg_ctx* c, size_t total_bytes, int n, int fmt) {
 
 // tables whose fill level the kernels report in the counter block
 bool tables_overflow(const fg_ctx* c, int fmt, const uint32_t* t) {
-    if (fmt == FG_FMT_RFC5424)
-        return t[fg::K5_ENTRIES] > c->e8_cap || t[fg::K5_ARENA] > c->arena_cap || t[fg::K5_WIDE_ROWS] > c->wide_cap ||
-               t[fg::K5_WIDE_ENTRIES] > c->entry_cap;
-    if (fmt == FG_FMT_RFC3164) return t[fg::K5_ARENA] > c->arena_cap;
-    return t[fg::K5_ENTRIES] > c->entry_cap;
+    for (const Table& tb : c->tables[fmt])
+        if (t[tb.slot] > tb.cols[0]->cap) return true;
+    return false;
 }
+// the allocators kept counting past the capacity: grow each overflowed table once to the exact need
 int regrow_tables(fg_ctx* c, int fmt, const uint32_t* t) {
-    auto grown = [](size_t need) { return need + need / 8 + 1024; };
-    if (fmt == FG_FMT_RFC5424) {
-        if (t[fg::K5_ENTRIES] > c->e8_cap)
-            if (int rc = alloc_e8(c, grown(t[fg::K5_ENTRIES]))) return rc;
-        if (t[fg::K5_ARENA] > c->arena_cap)
-            if (int rc = alloc_arena(c, grown(t[fg::K5_ARENA]))) return rc;
-        if (t[fg::K5_WIDE_ROWS] > c->wide_cap)
-            if (int rc = alloc_wide(c, grown(t[fg::K5_WIDE_ROWS]))) return rc;
-        if (t[fg::K5_WIDE_ENTRIES] > c->entry_cap)
-            if (int rc = alloc_entries(c, grown(t[fg::K5_WIDE_ENTRIES]))) return rc;
-        return FG_OK;
+    for (const Table& tb : c->tables[fmt]) {
+        const size_t need = t[tb.slot];
+        if (need > tb.cols[0]->cap)
+            for (Mirror* m : tb.cols) FG_CUDA(c, m->alloc(need + need / 8 + 1024));
     }
-    if (fmt == FG_FMT_RFC3164) return alloc_arena(c, grown(t[fg::K5_ARENA]));
-    return alloc_entries(c, grown(t[fg::K5_ENTRIES]));
+    return FG_OK;
 }
 
 // One parse launch over lines [line0, line0 + n) of the resident offsets (for RFC5424: parse + unescape + wide kernels)
@@ -423,25 +400,25 @@ int launch_lines(fg_ctx* c, int fmt, int line0, int n, int tile, const uint8_t* 
     if (fmt == FG_FMT_RFC5424) {
         fg::Parse5424Params P;
         P.bytes = c->d_bytes;
-        P.offsets = c->d_offsets + line0;
+        P.offsets = c->offsets.dev<int32_t>() + line0;
         P.n = n;
         P.tile_bytes = tile;
-        P.rows = c->d_rows5 + 2 * (size_t)line0;
-        P.entries = c->d_e8;
-        P.entry_cap = (uint32_t)std::min<size_t>(c->e8_cap, 0xFFFFFFFFu);
+        P.rows = c->rows5.dev<uint4>() + 2 * (size_t)line0;
+        P.entries = c->e8.dev<unsigned long long>();
+        P.entry_cap = cap32(c->e8);
         P.counters = c->d_k;
         P.esc_list = c->d_esc_list;
         P.wide_list = c->d_wide_list;
-        P.arena = c->d_arena;
-        P.arena_cap = (uint32_t)std::min<size_t>(c->arena_cap, 0xFFFFFFFFu);
-        P.wide_rows = c->d_wide;
-        P.wide_cap = (uint32_t)c->wide_cap;
-        P.wentry_name = c->d_entry_name;
-        P.wentry_val = c->d_entry_val;
-        P.wentry_meta = c->d_entry_meta;
-        P.wentry_cap = (uint32_t)std::min<size_t>(c->entry_cap, 0xFFFFFFFFu);
+        P.arena = c->arena.d;
+        P.arena_cap = cap32(c->arena);
+        P.wide_rows = c->wide.dev<fg::WideRow>();
+        P.wide_cap = cap32(c->wide);
+        P.wentry_name = c->entry_name.dev<int2>();
+        P.wentry_val = c->entry_val.dev<unsigned long long>();
+        P.wentry_meta = c->entry_meta.d;
+        P.wentry_cap = cap32(c->entry_name);
         P.line0 = line0;
-        P.bad_offsets = c->d_k + kBadFlag;
+        P.bad_offsets = c->d_k + fg::K5_BAD_OFFSETS;
         P.line_invalid = invalid;
         P.strip_eol = strip_eol;
         FG_CUDA(c, cudaMemsetAsync(c->d_k + fg::K5_ESC_LIST, 0, 8, s));  // the two work lists are per launch
@@ -451,11 +428,11 @@ int launch_lines(fg_ctx* c, int fmt, int line0, int n, int tile, const uint8_t* 
     }
     fg::ParseParams P;
     P.bytes = c->d_bytes;
-    P.offsets = c->d_offsets + line0;
+    P.offsets = c->offsets.dev<int32_t>() + line0;
     P.n = n;
     P.line0 = line0;
     P.tile_bytes = tile;
-    uint8_t* r = c->d_rows;
+    uint8_t* r = c->rows.d;
     P.ts = (double*)(r + col_off(c, C_TS)) + line0;
     P.meta = (uint32_t*)(r + col_off(c, C_META)) + line0;
     P.host = (int2*)(r + col_off(c, C_HOST)) + line0;
@@ -465,25 +442,25 @@ int launch_lines(fg_ctx* c, int fmt, int line0, int n, int tile, const uint8_t* 
     P.msg = (int2*)(r + col_off(c, C_MSG)) + line0;
     P.full = (int2*)(r + col_off(c, C_FULL)) + line0;
     P.sd = (int2*)(r + col_off(c, C_SD)) + line0;
-    P.entry_name = c->d_entry_name;
-    P.entry_val = c->d_entry_val;
-    P.entry_meta = c->d_entry_meta;
+    P.entry_name = c->entry_name.dev<int2>();
+    P.entry_val = c->entry_val.dev<unsigned long long>();
+    P.entry_meta = c->entry_meta.d;
     P.tmp_name = c->d_tmp_name;
     P.tmp_val = c->d_tmp_val;
     P.tmp_meta = c->d_tmp_meta;
     P.line_invalid = invalid;
     P.strip_eol = strip_eol;
     P.entry_counter = c->d_k + fg::K5_ENTRIES;
-    P.entry_cap = (uint32_t)std::min<size_t>(c->entry_cap, 0xFFFFFFFFu);
-    P.bad_offsets = c->d_k + kBadFlag;
+    P.entry_cap = cap32(c->entry_name);
+    P.bad_offsets = c->d_k + fg::K5_BAD_OFFSETS;
     P.slow_list = c->d_wide_list;
     P.slow_count = c->d_k + fg::K5_WIDE_LIST;
     if (fmt == FG_FMT_GELF) FG_CUDA(c, cudaMemsetAsync(c->d_k + fg::K5_WIDE_LIST, 0, 4, s));  // the work list is per launch
     P.ltsv = c->ltsv;
     P.r3164.year = c->call_year;
     P.r3164.tz = c->tz_dev;
-    P.r3164.arena = c->d_arena;
-    P.r3164.arena_cap = (uint32_t)std::min<size_t>(c->arena_cap, 0xFFFFFFFFu);
+    P.r3164.arena = c->arena.d;
+    P.r3164.arena_cap = cap32(c->arena);
     P.r3164.arena_counter = c->d_k + fg::K5_ARENA;
     if (time_dominant) FG_CUDA(c, cudaEventRecord(c->ev_dom0, s));
     FG_CUDA(c, fg::launch_parse(fmt, P, s));
@@ -496,25 +473,25 @@ bool col_used(int col) { return !(col == C_APP || col == C_PROC || col == C_MSGI
 
 void fill_out(fg_ctx* c, int fmt, int n, const uint32_t* tot, fg_batch_out* out) {
     out->n = n;
-    out->entry_name = c->h_entry_name;
-    out->entry_val = c->h_entry_val;
-    out->entry_meta = c->h_entry_meta;
+    out->entry_name = c->entry_name.host<fg_span>();
+    out->entry_val = c->entry_val.host<uint64_t>();
+    out->entry_meta = c->entry_meta.h;
     if (fmt == FG_FMT_RFC5424) {
         out->n_entries = (int32_t)tot[fg::K5_WIDE_ENTRIES];
-        out->rows5424 = c->h_rows5;
-        out->entries8 = c->h_e8;
+        out->rows5424 = c->rows5.host<fg_row5424>();
+        out->entries8 = c->e8.host<uint64_t>();
         out->n_entries8 = (int32_t)tot[fg::K5_ENTRIES];
         out->n_wide = (int32_t)tot[fg::K5_WIDE_ROWS];
-        out->wide_rows = c->h_wide;
-        out->arena = c->h_arena;
+        out->wide_rows = c->wide.host<fg_wide_row>();
+        out->arena = c->arena.h;
         out->arena_bytes = (int64_t)tot[fg::K5_ARENA];
         return;
     }
-    uint8_t* r = c->h_rows;
+    uint8_t* r = c->rows.h;
     out->n_entries = (int32_t)tot[fg::K5_ENTRIES];
     if (fmt == FG_FMT_RFC3164) {
         out->n_entries = 0;
-        out->arena = c->h_arena;
+        out->arena = c->arena.h;
         out->arena_bytes = (int64_t)tot[fg::K5_ARENA];
     }
     out->ts = (const double*)(r + col_off(c, C_TS));
@@ -528,14 +505,14 @@ void fill_out(fg_ctx* c, int fmt, int n, const uint32_t* tot, fg_batch_out* out)
 int copy_rows_d2h(fg_ctx* c, int fmt, int line0, int n, cudaStream_t s) {
     if (n <= 0) return FG_OK;
     if (fmt == FG_FMT_RFC5424) {
-        FG_CUDA(c, cudaMemcpyAsync(c->h_rows5 + line0, c->d_rows5 + 2 * (size_t)line0, (size_t)n * 32, cudaMemcpyDeviceToHost, s));
+        FG_CUDA(c, c->rows5.d2h(line0, line0 + n, s));
         return FG_OK;
     }
     // ts and meta: one copy each; the 8-byte span columns share one pitch (8 * max_lines), so every run of consecutive
     // used span columns goes back as ONE 2-D copy (few large D2H operations disturb the concurrent H2D stream less)
     for (int col = C_TS; col <= C_META; ++col) {
         const size_t o = col_off(c, col) + (size_t)line0 * kColW[col];
-        FG_CUDA(c, cudaMemcpyAsync(c->h_rows + o, c->d_rows + o, (size_t)n * kColW[col], cudaMemcpyDeviceToHost, s));
+        FG_CUDA(c, c->rows.d2h(o, o + (size_t)n * kColW[col], s));
     }
     const size_t pitch = (size_t)c->max_lines * 8;
     int col = C_HOST;
@@ -544,41 +521,18 @@ int copy_rows_d2h(fg_ctx* c, int fmt, int line0, int n, cudaStream_t s) {
         int end = col;
         while (end + 1 < C_COUNT && col_used(end + 1)) ++end;
         const size_t o = col_off(c, col) + (size_t)line0 * 8;
-        FG_CUDA(c, cudaMemcpy2DAsync(c->h_rows + o, pitch, c->d_rows + o, pitch, (size_t)n * 8, (size_t)(end - col + 1),
+        FG_CUDA(c, cudaMemcpy2DAsync(c->rows.h + o, pitch, c->rows.d + o, pitch, (size_t)n * 8, (size_t)(end - col + 1),
                                      cudaMemcpyDeviceToHost, s));
         col = end + 1;
     }
     return FG_OK;
 }
 
-int copy_entries_range(fg_ctx* c, size_t from, size_t to, cudaStream_t s) {
-    if (to <= from) return FG_OK;
-    const size_t k = to - from;
-    FG_CUDA(c, cudaMemcpyAsync(c->h_entry_name + from, c->d_entry_name + from, k * sizeof(int2), cudaMemcpyDeviceToHost, s));
-    FG_CUDA(c, cudaMemcpyAsync(c->h_entry_val + from, c->d_entry_val + from, k * sizeof(uint64_t), cudaMemcpyDeviceToHost, s));
-    FG_CUDA(c, cudaMemcpyAsync(c->h_entry_meta + from, c->d_entry_meta + from, k, cudaMemcpyDeviceToHost, s));
+// side tables on s_d2h: the rows a parse step produced are the contiguous range [prev, cur) of each bump allocator
+int copy_tables_d2h(fg_ctx* c, int fmt, const uint32_t* prev, const uint32_t* cur) {
+    for (const Table& tb : c->tables[fmt])
+        for (const Mirror* m : tb.cols) FG_CUDA(c, m->d2h(prev[tb.slot], cur[tb.slot], c->s_d2h));
     return FG_OK;
-}
-
-// side tables: the rows a chunk produced are the contiguous range [prev, cur) of each bump allocator
-int copy_tables_d2h(fg_ctx* c, int fmt, const uint32_t* prev, const uint32_t* cur, cudaStream_t s) {
-    if (fmt == FG_FMT_RFC3164) {
-        if (cur[fg::K5_ARENA] > prev[fg::K5_ARENA])
-            FG_CUDA(c, cudaMemcpyAsync(c->h_arena + prev[fg::K5_ARENA], c->d_arena + prev[fg::K5_ARENA],
-                                       (size_t)(cur[fg::K5_ARENA] - prev[fg::K5_ARENA]), cudaMemcpyDeviceToHost, s));
-        return FG_OK;
-    }
-    if (fmt != FG_FMT_RFC5424) return copy_entries_range(c, prev[fg::K5_ENTRIES], cur[fg::K5_ENTRIES], s);
-    if (cur[fg::K5_ENTRIES] > prev[fg::K5_ENTRIES])
-        FG_CUDA(c, cudaMemcpyAsync(c->h_e8 + prev[fg::K5_ENTRIES], c->d_e8 + prev[fg::K5_ENTRIES],
-                                   (size_t)(cur[fg::K5_ENTRIES] - prev[fg::K5_ENTRIES]) * 8, cudaMemcpyDeviceToHost, s));
-    if (cur[fg::K5_ARENA] > prev[fg::K5_ARENA])
-        FG_CUDA(c, cudaMemcpyAsync(c->h_arena + prev[fg::K5_ARENA], c->d_arena + prev[fg::K5_ARENA],
-                                   (size_t)(cur[fg::K5_ARENA] - prev[fg::K5_ARENA]), cudaMemcpyDeviceToHost, s));
-    if (cur[fg::K5_WIDE_ROWS] > prev[fg::K5_WIDE_ROWS])
-        FG_CUDA(c, cudaMemcpyAsync(c->h_wide + prev[fg::K5_WIDE_ROWS], c->d_wide + prev[fg::K5_WIDE_ROWS],
-                                   (size_t)(cur[fg::K5_WIDE_ROWS] - prev[fg::K5_WIDE_ROWS]) * sizeof(fg_wide_row), cudaMemcpyDeviceToHost, s));
-    return copy_entries_range(c, prev[fg::K5_WIDE_ENTRIES], cur[fg::K5_WIDE_ENTRIES], s);
 }
 
 bool is_pinned(const void* p) {
@@ -625,8 +579,82 @@ int ensure_events(fg_ctx* c, int chunks) {
     }
     if (c->h_counts_cap < chunks) {
         hfree(c->h_counts);
-        FG_CUDA(c, cudaHostAlloc(&c->h_counts, sizeof(uint32_t) * kCnt * (size_t)chunks, cudaHostAllocDefault));
+        FG_CUDA(c, cudaHostAlloc(&c->h_counts, sizeof(uint32_t) * fg::K5_COUNT * (size_t)chunks, cudaHostAllocDefault));
         c->h_counts_cap = chunks;
+    }
+    return FG_OK;
+}
+
+// A caller's batch on its way to the device, chunk by chunk
+struct Input {
+    const uint8_t* bytes;
+    const int32_t* offsets;
+    bool pin_b, pin_o;
+    int bounce_ix;
+};
+
+// Chunk k = lines [l0, l1) of a caller's batch: H2D of its bytes and offsets, then on s_comp the offsets check and,
+// after ev_k0[k], the parse.
+int enqueue_chunk(fg_ctx* c, int fmt, Input& in, int k, int l0, int l1, int tile) {
+    const size_t b0 = (size_t)in.offsets[l0], b1 = (size_t)in.offsets[l1];
+    if (b1 < b0 || b1 > c->max_bytes) {
+        cudaDeviceSynchronize();
+        return fail(c, FG_E_ARG, kBadOffsets);
+    }
+    int32_t* d_offsets = c->offsets.dev<int32_t>();
+    if (int rc = h2d(c, c->d_bytes + b0, in.bytes + b0, b1 - b0, in.pin_b, in.bounce_ix)) return rc;
+    if (int rc = h2d(c, d_offsets + l0, in.offsets + l0, sizeof(int32_t) * (size_t)(l1 - l0 + 1), in.pin_o, in.bounce_ix)) return rc;
+    FG_CUDA(c, cudaEventRecord(c->ev_h2d[k], c->s_h2d));
+    FG_CUDA(c, cudaStreamWaitEvent(c->s_comp, c->ev_h2d[k], 0));
+    FG_CUDA(c, fg::launch_check_offsets(d_offsets + l0, l1 - l0, (long long)c->max_bytes, c->d_k + fg::K5_BAD_OFFSETS, c->s_comp));
+    FG_CUDA(c, cudaEventRecord(c->ev_k0[k], c->s_comp));
+    return launch_lines(c, fmt, l0, l1 - l0, tile, nullptr, 0, c->s_comp);
+}
+
+// Ends parse step j on stream s: ev_k1[j] closes its kernel time, the counter block is snapshotted into h_counts (with
+// element j + 1 of `running`, if given), ev_cnt[j] marks the snapshot, and s_d2h waits for it before the step's
+// results are copied back.
+int end_step(fg_ctx* c, int j, cudaStream_t s, const Mirror* running = nullptr) {
+    FG_CUDA(c, cudaEventRecord(c->ev_k1[j], s));
+    FG_CUDA(c, cudaMemcpyAsync(c->h_counts + (size_t)j * fg::K5_COUNT, c->d_k, sizeof(uint32_t) * fg::K5_COUNT, cudaMemcpyDeviceToHost, s));
+    if (running) FG_CUDA(c, running->d2h(j + 1, j + 2, s));
+    FG_CUDA(c, cudaEventRecord(c->ev_cnt[j], s));
+    FG_CUDA(c, cudaStreamWaitEvent(c->s_d2h, c->ev_cnt[j], 0));
+    return FG_OK;
+}
+
+// Drains parse steps [0, steps) of one attempt, in order.  As soon as step j's counters arrive, `copy(j, prev, cur)`
+// enqueues what step j produced on s_d2h while later steps are still in flight; it returns kRedo when a range of its
+// own does not fit.  After an overflow nothing more is copied: the overflowed tables are grown to the exact need and
+// kRedo asks the caller to enqueue the attempt again.  Otherwise *kms is the summed kernel time of the steps.
+// total receives the last snapshot.
+template <class Copy>
+int drain(fg_ctx* c, int fmt, int steps, Copy&& copy, uint32_t* total, float* kms) {
+    uint32_t prev[fg::K5_COUNT] = {};
+    memset(total, 0, sizeof prev);
+    bool overflow = false;
+    for (int j = 0; j < steps; ++j) {
+        FG_CUDA(c, cudaEventSynchronize(c->ev_cnt[j]));
+        const uint32_t* cur = c->h_counts + (size_t)j * fg::K5_COUNT;
+        memcpy(total, cur, sizeof prev);
+        overflow = overflow || tables_overflow(c, fmt, cur);
+        if (overflow) continue;  // keep draining the events; the attempt is redone below
+        const int rc = copy(j, prev, cur);
+        if (rc == kRedo) overflow = true;
+        else if (rc) return rc;
+        memcpy(prev, cur, sizeof prev);
+    }
+    FG_CUDA(c, cudaStreamSynchronize(c->s_d2h));
+    if (total[fg::K5_BAD_OFFSETS]) return fail(c, FG_E_ARG, kBadOffsets);
+    if (overflow) {
+        if (int rc = regrow_tables(c, fmt, total)) return rc;
+        return kRedo;
+    }
+    *kms = 0.f;
+    for (int j = 0; j < steps; ++j) {
+        float ms = 0.f;
+        FG_CUDA(c, cudaEventElapsedTime(&ms, c->ev_k0[j], c->ev_k1[j]));
+        *kms += ms;
     }
     return FG_OK;
 }
@@ -704,31 +732,14 @@ int build_static_items(fg_ctx* c) {
         lit_off.push_back((int32_t)blob.size());
         kind.push_back(it.kind);
     }
-    const size_t n = items.size();
-    const size_t o_key = (blob.size() + 15) & ~(size_t)15, o_lit = o_key + (n + 1) * 4, o_kind = o_lit + (n + 1) * 4;
-    std::vector<uint8_t> buf(o_kind + n * 4 + 16, 0);
-    memcpy(buf.data(), blob.data(), blob.size());
-    memcpy(buf.data() + o_key, key_off.data(), (n + 1) * 4);
-    memcpy(buf.data() + o_lit, lit_off.data(), (n + 1) * 4);
-    memcpy(buf.data() + o_kind, kind.data(), n * 4);
-    dfree(c->d_static_blob);
-    FG_CUDA(c, cudaMalloc(&c->d_static_blob, buf.size()));
-    FG_CUDA(c, cudaMemcpy(c->d_static_blob, buf.data(), buf.size(), cudaMemcpyHostToDevice));
-    c->n_static = (int)n;
+    Blob b;
+    b.put(blob);  // at offset 0: d_static_blob is the base of key_off / lit_off
+    const size_t o_key = b.put(key_off), o_lit = b.put(lit_off), o_kind = b.put(kind);
+    FG_CUDA(c, b.upload(c->d_static_blob));
+    c->n_static = (int)items.size();
     c->d_static_key_off = (const int32_t*)(c->d_static_blob + o_key);
     c->d_static_lit_off = (const int32_t*)(c->d_static_blob + o_lit);
     c->d_static_kind = (const int32_t*)(c->d_static_blob + o_kind);
-    return FG_OK;
-}
-
-int alloc_enc_out(fg_ctx* c, size_t cap) {
-    dfree(c->d_enc_out);
-    hfree(c->h_enc_out);
-    c->enc_out_cap = 0;
-    cap = (cap + 4095) & ~(size_t)4095;
-    FG_CUDA(c, cudaMalloc(&c->d_enc_out, cap + 16));
-    FG_CUDA(c, cudaHostAlloc(&c->h_enc_out, cap + 16, cudaHostAllocDefault));
-    c->enc_out_cap = cap;
     return FG_OK;
 }
 
@@ -736,22 +747,13 @@ int ensure_encoder(fg_ctx* c, int chunks) {
     if (!c->d_enc_lens) {
         FG_CUDA(c, cudaMalloc(&c->d_enc_lens, (size_t)c->max_lines * 4));
         FG_CUDA(c, cudaMalloc(&c->d_enc_rel, (size_t)c->max_lines * 4));
-        FG_CUDA(c, cudaMalloc(&c->d_enc_offsets, ((size_t)c->max_lines + 1) * 8));
-        FG_CUDA(c, cudaHostAlloc(&c->h_enc_offsets, ((size_t)c->max_lines + 1) * 8, cudaHostAllocDefault));
-        FG_CUDA(c, cudaMalloc(&c->d_enc_status, (size_t)c->max_lines));
-        FG_CUDA(c, cudaHostAlloc(&c->h_enc_status, (size_t)c->max_lines, cudaHostAllocDefault));
+        FG_CUDA(c, c->enc_offsets.alloc((size_t)c->max_lines + 1));
+        FG_CUDA(c, c->enc_status.alloc(c->max_lines));
         c->scan_temp_bytes = fg::gelf_scan_temp_bytes(c->max_lines);
         FG_CUDA(c, cudaMalloc(&c->d_scan_temp, c->scan_temp_bytes + 256));
     }
-    if (!c->enc_out_cap)
-        if (int rc = alloc_enc_out(c, c->max_bytes * 2 + (size_t)c->max_lines * 200)) return rc;
-    if (c->enc_base_cap < chunks + 1) {
-        dfree(c->d_enc_base);
-        hfree(c->h_enc_base);
-        FG_CUDA(c, cudaMalloc(&c->d_enc_base, sizeof(unsigned long long) * ((size_t)chunks + 1)));
-        FG_CUDA(c, cudaHostAlloc(&c->h_enc_base, sizeof(unsigned long long) * ((size_t)chunks + 1), cudaHostAllocDefault));
-        c->enc_base_cap = chunks + 1;
-    }
+    if (!c->enc_out.cap) FG_CUDA(c, c->enc_out.alloc(c->max_bytes * 2 + (size_t)c->max_lines * 200));
+    if (c->enc_base.cap < (size_t)chunks + 1) FG_CUDA(c, c->enc_base.alloc((size_t)chunks + 1));
     if (!c->d_static_blob)
         if (int rc = build_static_items(c)) return rc;
     return FG_OK;
@@ -783,7 +785,8 @@ int fg_create(const fg_config* cfg, fg_ctx** out) {
     c->chunk_lines = (c->chunk_lines + 127) / 128 * 128;  // a multiple of every kernel's lines per CTA
     c->r3164_year = cfg->rfc3164_year;
     if (cfg->tzdir) c->tzdir = cfg->tzdir;
-#define FG_CREATE_CUDA(call)                                  \
+    list_tables(c);
+#define FG_CREATE_CUDA(call)                                 \
     do {                                                      \
         cudaError_t _e = (call);                              \
         if (_e != cudaSuccess) {                              \
@@ -808,7 +811,7 @@ int fg_create(const fg_config* cfg, fg_ctx** out) {
     FG_CREATE_CUDA(cudaEventCreate(&c->ev_dom1));
     FG_CREATE_CUDA(cudaMalloc(&c->d_bytes, c->max_bytes + kPad));
     FG_CREATE_CUDA(cudaMemset(c->d_bytes + c->max_bytes, 0, kPad));
-    FG_CREATE_CUDA(cudaMalloc(&c->d_offsets, sizeof(int32_t) * ((size_t)c->max_lines + 1)));
+    FG_CREATE_CUDA(c->offsets.alloc((size_t)c->max_lines + 1));
     FG_CREATE_CUDA(cudaMalloc(&c->d_k, 256));
     FG_CREATE_CUDA(cudaMemset(c->d_k, 0, 256));
     for (int b = 0; b < 2; ++b) {
@@ -839,17 +842,9 @@ int fg_create(const fg_config* cfg, fg_ctx** out) {
             }
             L.suffix_off[t + 1] = (int32_t)suffix.size();
         }
-        const size_t o_names = 0, o_off = (names.size() + 15) & ~(size_t)15;
-        const size_t o_types = o_off + ((name_off.size() * 4 + 15) & ~(size_t)15);
-        const size_t o_suf = o_types + ((types.size() * 4 + 15) & ~(size_t)15);
-        const size_t total = o_suf + suffix.size() + 16;
-        std::vector<uint8_t> blob(total, 0);
-        if (!names.empty()) memcpy(blob.data() + o_names, names.data(), names.size());
-        memcpy(blob.data() + o_off, name_off.data(), name_off.size() * 4);
-        if (!types.empty()) memcpy(blob.data() + o_types, types.data(), types.size() * 4);
-        if (!suffix.empty()) memcpy(blob.data() + o_suf, suffix.data(), suffix.size());
-        FG_CREATE_CUDA(cudaMalloc(&c->d_ltsv_blob, total));
-        FG_CREATE_CUDA(cudaMemcpy(c->d_ltsv_blob, blob.data(), total, cudaMemcpyHostToDevice));
+        Blob b;
+        const size_t o_names = b.put(names), o_off = b.put(name_off), o_types = b.put(types), o_suf = b.put(suffix);
+        FG_CREATE_CUDA(b.upload(c->d_ltsv_blob));
         L.names = c->d_ltsv_blob + o_names;
         L.name_off = (const int32_t*)(c->d_ltsv_blob + o_off);
         L.types = (const int32_t*)(c->d_ltsv_blob + o_types);
@@ -864,25 +859,19 @@ void fg_destroy(fg_ctx* c) {
     if (!c) return;
     cudaSetDevice(c->device);
     cudaDeviceSynchronize();
-    dfree(c->d_entry_name); dfree(c->d_entry_val); dfree(c->d_entry_meta);
-    hfree(c->h_entry_name); hfree(c->h_entry_val); hfree(c->h_entry_meta);
-    dfree(c->d_bytes); dfree(c->d_offsets); dfree(c->d_rows); dfree(c->d_k); dfree(c->d_flush);
-    dfree(c->d_rows5); hfree(c->h_rows5); dfree(c->d_e8); hfree(c->h_e8); dfree(c->d_esc_list); dfree(c->d_wide_list);
-    dfree(c->d_arena); hfree(c->h_arena); dfree(c->d_wide); hfree(c->h_wide);
-    dfree(c->d_enc_lens); dfree(c->d_enc_rel); dfree(c->d_enc_base); hfree(c->h_enc_base); dfree(c->d_enc_out); hfree(c->h_enc_out);
-    dfree(c->d_enc_offsets); hfree(c->h_enc_offsets); dfree(c->d_enc_status); hfree(c->h_enc_status); dfree(c->d_scan_temp);
+    dfree(c->d_bytes); dfree(c->d_k); dfree(c->d_flush); dfree(c->d_esc_list); dfree(c->d_wide_list);
+    dfree(c->d_enc_lens); dfree(c->d_enc_rel); dfree(c->d_scan_temp);
     dfree(c->d_static_blob);
     dfree(c->d_seg); dfree(c->d_n_lines); dfree(c->d_invalid);
-    hfree(c->h_offsets); hfree(c->h_n_lines);
+    hfree(c->h_n_lines);
     if (c->s_parse) cudaStreamDestroy(c->s_parse);
     for (auto e : c->ev_split) cudaEventDestroy(e);
-    dfree(c->d_cum); hfree(c->h_cum);
     if (c->ev_s0) cudaEventDestroy(c->ev_s0);
     if (c->ev_s1) cudaEventDestroy(c->ev_s1);
     dfree(c->d_tmp_name); dfree(c->d_tmp_val); dfree(c->d_tmp_meta);
     dfree(c->d_ltsv_blob);
     dfree(c->d_tz_blob);
-    hfree(c->h_rows); hfree(c->h_counts);
+    hfree(c->h_counts);
     for (int b = 0; b < 2; ++b) {
         hfree(c->h_bounce[b]);
         if (c->bounce_ev[b]) cudaEventDestroy(c->bounce_ev[b]);
@@ -898,7 +887,7 @@ void fg_destroy(fg_ctx* c) {
     if (c->s_h2d) cudaStreamDestroy(c->s_h2d);
     if (c->s_comp) cudaStreamDestroy(c->s_comp);
     if (c->s_d2h) cudaStreamDestroy(c->s_d2h);
-    delete c;
+    delete c;  // the mirrors release themselves
 }
 
 const char* fg_last_error(const fg_ctx* c) { return c ? c->last_error.c_str() : "null context"; }
@@ -922,72 +911,32 @@ int fg_decode_batch(fg_ctx* c, fg_format fmt, const uint8_t* bytes, const int32_
     if (int rc = ensure_format(c, (int)fmt)) return rc;
     c->call_year = current_year(c);
     memset(out, 0, sizeof *out);
-    const uint32_t zero[kCnt] = {};
+    const uint32_t zero[fg::K5_COUNT] = {};
     if (n == 0) {
         fill_out(c, fmt, 0, zero, out);
         return FG_OK;
     }
     const auto t_begin = std::chrono::steady_clock::now();
-    const bool pin_b = is_pinned(bytes), pin_o = is_pinned(offsets);
+    Input in{bytes, offsets, is_pinned(bytes), is_pinned(offsets), 0};
     const int C = c->chunk_lines;
     const int chunks = (n + C - 1) / C;
     if (int rc = ensure_events(c, chunks)) return rc;
     const int tile = pick_tile(c, (size_t)(offsets[n] - offsets[0]), n, (int)fmt);
+    auto copy_tables = [&](int, const uint32_t* prev, const uint32_t* cur) { return copy_tables_d2h(c, fmt, prev, cur); };
     for (int attempt = 0; attempt < 2; ++attempt) {
-        FG_CUDA(c, cudaMemsetAsync(c->d_k, 0, sizeof(uint32_t) * kCnt, c->s_comp));
-        int bounce_ix = 0;
+        FG_CUDA(c, cudaMemsetAsync(c->d_k, 0, sizeof(uint32_t) * fg::K5_COUNT, c->s_comp));
+        in.bounce_ix = 0;
         for (int k = 0; k < chunks; ++k) {
             const int l0 = k * C, l1 = std::min(n, l0 + C);
-            const size_t b0 = (size_t)offsets[l0], b1 = (size_t)offsets[l1];
-            if (b1 < b0 || b1 > c->max_bytes) {
-                cudaDeviceSynchronize();
-                return fail(c, FG_E_ARG, "offsets must be non-decreasing and within max_batch_bytes");
-            }
-            if (int rc = h2d(c, c->d_bytes + b0, bytes + b0, b1 - b0, pin_b, bounce_ix)) return rc;
-            if (int rc = h2d(c, c->d_offsets + l0, offsets + l0, sizeof(int32_t) * (size_t)(l1 - l0 + 1), pin_o, bounce_ix))
-                return rc;
-            FG_CUDA(c, cudaEventRecord(c->ev_h2d[k], c->s_h2d));
-            FG_CUDA(c, cudaStreamWaitEvent(c->s_comp, c->ev_h2d[k], 0));
-            FG_CUDA(c, fg::launch_check_offsets(c->d_offsets + l0, l1 - l0, (long long)c->max_bytes, c->d_k + kBadFlag, c->s_comp));
-            FG_CUDA(c, cudaEventRecord(c->ev_k0[k], c->s_comp));
-            if (int rc = launch_lines(c, (int)fmt, l0, l1 - l0, tile, nullptr, 0, c->s_comp)) return rc;
-            FG_CUDA(c, cudaEventRecord(c->ev_k1[k], c->s_comp));
-            FG_CUDA(c, cudaMemcpyAsync(c->h_counts + (size_t)k * kCnt, c->d_k, sizeof(uint32_t) * kCnt, cudaMemcpyDeviceToHost, c->s_comp));
-            FG_CUDA(c, cudaEventRecord(c->ev_cnt[k], c->s_comp));
-            FG_CUDA(c, cudaStreamWaitEvent(c->s_d2h, c->ev_cnt[k], 0));
+            if (int rc = enqueue_chunk(c, fmt, in, k, l0, l1, tile)) return rc;
+            if (int rc = end_step(c, k, c->s_comp)) return rc;
             if (int rc = copy_rows_d2h(c, fmt, l0, l1 - l0, c->s_d2h)) return rc;
         }
-        // side tables: chunk k's rows are the contiguous range [count(k-1), count(k)) of each bump allocator; a range is
-        // copied back as soon as its chunk has been parsed, while later chunks are still in flight
-        uint32_t prev[kCnt] = {};
-        bool overflow = false;
-        for (int k = 0; k < chunks; ++k) {
-            FG_CUDA(c, cudaEventSynchronize(c->ev_cnt[k]));
-            const uint32_t* cur = c->h_counts + (size_t)k * kCnt;
-            if (tables_overflow(c, (int)fmt, cur)) {
-                overflow = true;
-                continue;  // keep draining the events; the batch is redone below
-            }
-            if (!overflow) {
-                if (int rc = copy_tables_d2h(c, (int)fmt, prev, cur, c->s_d2h)) return rc;
-                memcpy(prev, cur, sizeof prev);
-            }
-        }
-        uint32_t total[kCnt];
-        memcpy(total, c->h_counts + (size_t)(chunks - 1) * kCnt, sizeof total);
-        FG_CUDA(c, cudaStreamSynchronize(c->s_d2h));
-        if (total[kBadFlag]) return fail(c, FG_E_ARG, "offsets must be non-decreasing and within max_batch_bytes");
-        if (overflow) {
-            // the allocators kept counting past the capacity: grow once to the exact need and redo
-            if (int rc = regrow_tables(c, (int)fmt, total)) return rc;
-            continue;
-        }
+        uint32_t total[fg::K5_COUNT];
         float kms = 0.f;
-        for (int k = 0; k < chunks; ++k) {
-            float ms = 0.f;
-            FG_CUDA(c, cudaEventElapsedTime(&ms, c->ev_k0[k], c->ev_k1[k]));
-            kms += ms;
-        }
+        const int rc = drain(c, fmt, chunks, copy_tables, total, &kms);
+        if (rc == kRedo) continue;
+        if (rc) return rc;
         fill_out(c, fmt, n, total, out);
         out->kernel_ms = kms;
         out->total_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t_begin).count();
@@ -1089,46 +1038,43 @@ int fg_decode_encode_gelf(fg_ctx* c, fg_format fmt, const uint8_t* bytes, const 
     const int chunks = n > 0 ? (n + C - 1) / C : 1;
     if (int rc = ensure_encoder(c, chunks)) return rc;
     memset(out, 0, sizeof *out);
-    out->bytes = c->h_enc_out;
-    out->offsets = c->h_enc_offsets;
-    out->status = c->h_enc_status;
+    out->bytes = c->enc_out.h;
+    out->offsets = c->enc_offsets.host<int64_t>();
+    out->status = c->enc_status.h;
     if (n == 0) {
-        c->h_enc_offsets[0] = 0;
+        c->enc_offsets.host<int64_t>()[0] = 0;
         return FG_OK;
     }
     const auto t_begin = std::chrono::steady_clock::now();
-    const bool pin_b = is_pinned(bytes), pin_o = is_pinned(offsets);
+    Input in{bytes, offsets, is_pinned(bytes), is_pinned(offsets), 0};
     if (int rc = ensure_events(c, chunks)) return rc;
     const int tile = pick_tile(c, (size_t)(offsets[n] - offsets[0]), n, (int)fmt);
+    // encoded bytes: chunk k's records are the contiguous range [base(k), base(k+1)) of the output
+    unsigned long long* base = c->enc_base.host<unsigned long long>();
+    base[0] = 0;
+    auto copy_records = [&](int k, const uint32_t*, const uint32_t*) {
+        if (base[k + 1] > c->enc_out.cap) return kRedo;
+        FG_CUDA(c, c->enc_out.d2h(base[k], base[k + 1], c->s_d2h));
+        return FG_OK;
+    };
     for (int attempt = 0; attempt < 3; ++attempt) {
-        FG_CUDA(c, cudaMemsetAsync(c->d_k, 0, sizeof(uint32_t) * kCnt, c->s_comp));
-        FG_CUDA(c, cudaMemsetAsync(c->d_enc_base, 0, sizeof(unsigned long long), c->s_comp));
-        int bounce_ix = 0;
+        FG_CUDA(c, cudaMemsetAsync(c->d_k, 0, sizeof(uint32_t) * fg::K5_COUNT, c->s_comp));
+        FG_CUDA(c, cudaMemsetAsync(c->enc_base.d, 0, sizeof(unsigned long long), c->s_comp));
+        in.bounce_ix = 0;
         for (int k = 0; k < chunks; ++k) {
             const int l0 = k * C, l1 = std::min(n, l0 + C);
-            const size_t b0 = (size_t)offsets[l0], b1 = (size_t)offsets[l1];
-            if (b1 < b0 || b1 > c->max_bytes) {
-                cudaDeviceSynchronize();
-                return fail(c, FG_E_ARG, "offsets must be non-decreasing and within max_batch_bytes");
-            }
-            if (int rc = h2d(c, c->d_bytes + b0, bytes + b0, b1 - b0, pin_b, bounce_ix)) return rc;
-            if (int rc = h2d(c, c->d_offsets + l0, offsets + l0, sizeof(int32_t) * (size_t)(l1 - l0 + 1), pin_o, bounce_ix)) return rc;
-            FG_CUDA(c, cudaEventRecord(c->ev_h2d[k], c->s_h2d));
-            FG_CUDA(c, cudaStreamWaitEvent(c->s_comp, c->ev_h2d[k], 0));
-            FG_CUDA(c, fg::launch_check_offsets(c->d_offsets + l0, l1 - l0, (long long)c->max_bytes, c->d_k + kBadFlag, c->s_comp));
-            FG_CUDA(c, cudaEventRecord(c->ev_k0[k], c->s_comp));
-            if (int rc = launch_lines(c, (int)fmt, l0, l1 - l0, tile, nullptr, 0, c->s_comp)) return rc;
+            if (int rc = enqueue_chunk(c, fmt, in, k, l0, l1, tile)) return rc;
             fg::GelfEncodeParams E;
             E.bytes = c->d_bytes;
-            E.offsets = c->d_offsets + l0;
+            E.offsets = c->offsets.dev<int32_t>() + l0;
             E.n = l1 - l0;
-            E.rows = c->d_rows5 + 2 * (size_t)l0;
-            E.entries = c->d_e8;
-            E.arena = c->d_arena;
-            E.wide_rows = c->d_wide;
-            E.wentry_name = c->d_entry_name;
-            E.wentry_val = c->d_entry_val;
-            E.wentry_meta = c->d_entry_meta;
+            E.rows = c->rows5.dev<uint4>() + 2 * (size_t)l0;
+            E.entries = c->e8.dev<unsigned long long>();
+            E.arena = c->arena.d;
+            E.wide_rows = c->wide.dev<fg::WideRow>();
+            E.wentry_name = c->entry_name.dev<int2>();
+            E.wentry_val = c->entry_val.dev<unsigned long long>();
+            E.wentry_meta = c->entry_meta.d;
             E.static_blob = c->d_static_blob;
             E.n_static = c->n_static;
             E.static_key_off = c->d_static_key_off;
@@ -1136,56 +1082,32 @@ int fg_decode_encode_gelf(fg_ctx* c, fg_format fmt, const uint8_t* bytes, const 
             E.static_kind = c->d_static_kind;
             E.lens = c->d_enc_lens + l0;
             E.rel = c->d_enc_rel + l0;
-            E.base = c->d_enc_base + k;
-            E.out = c->d_enc_out;
-            E.out_cap = c->enc_out_cap;
-            E.out_offsets = c->d_enc_offsets + l0;
-            E.status = c->d_enc_status + l0;
-            E.bad_offsets = c->d_k + kBadFlag;
-            E.entry_cap = (uint32_t)std::min<size_t>(c->e8_cap, 0xFFFFFFFFu);
-            E.wide_cap = (uint32_t)c->wide_cap;
-            E.wentry_cap = (uint32_t)std::min<size_t>(c->entry_cap, 0xFFFFFFFFu);
+            E.base = c->enc_base.dev<unsigned long long>() + k;
+            E.out = c->enc_out.d;
+            E.out_cap = c->enc_out.cap;
+            E.out_offsets = c->enc_offsets.dev<long long>() + l0;
+            E.status = c->enc_status.d + l0;
+            E.bad_offsets = c->d_k + fg::K5_BAD_OFFSETS;
+            E.entry_cap = cap32(c->e8);
+            E.wide_cap = cap32(c->wide);
+            E.wentry_cap = cap32(c->entry_name);
             E.tile_bytes = std::min(4 * tile, c->max_tile5);  // the encoder's CTAs take 256 lines (4 x the parse kernel's 64)
             FG_CUDA(c, fg::launch_gelf_encode(E, c->d_scan_temp, c->scan_temp_bytes, c->s_comp));
             c->launches += 4;
-            FG_CUDA(c, cudaEventRecord(c->ev_k1[k], c->s_comp));
-            FG_CUDA(c, cudaMemcpyAsync(c->h_counts + (size_t)k * kCnt, c->d_k, sizeof(uint32_t) * kCnt, cudaMemcpyDeviceToHost, c->s_comp));
-            FG_CUDA(c, cudaMemcpyAsync(c->h_enc_base + k + 1, c->d_enc_base + k + 1, sizeof(unsigned long long), cudaMemcpyDeviceToHost, c->s_comp));
-            FG_CUDA(c, cudaEventRecord(c->ev_cnt[k], c->s_comp));
-            FG_CUDA(c, cudaStreamWaitEvent(c->s_d2h, c->ev_cnt[k], 0));
-            FG_CUDA(c, cudaMemcpyAsync(c->h_enc_status + l0, c->d_enc_status + l0, (size_t)(l1 - l0), cudaMemcpyDeviceToHost, c->s_d2h));
-            FG_CUDA(c, cudaMemcpyAsync(c->h_enc_offsets + l0, c->d_enc_offsets + l0, (size_t)(l1 - l0 + 1) * 8, cudaMemcpyDeviceToHost, c->s_d2h));
+            if (int rc = end_step(c, k, c->s_comp, &c->enc_base)) return rc;
+            FG_CUDA(c, c->enc_status.d2h(l0, l1, c->s_d2h));
+            FG_CUDA(c, c->enc_offsets.d2h(l0, l1 + 1, c->s_d2h));
         }
-        // encoded bytes: chunk k's records are the contiguous range [base(k), base(k+1)) of the output
-        c->h_enc_base[0] = 0;
-        bool overflow = false;
-        for (int k = 0; k < chunks; ++k) {
-            FG_CUDA(c, cudaEventSynchronize(c->ev_cnt[k]));
-            const uint32_t* cur = c->h_counts + (size_t)k * kCnt;
-            const unsigned long long lo = c->h_enc_base[k], hi = c->h_enc_base[k + 1];
-            if (tables_overflow(c, (int)fmt, cur) || hi > c->enc_out_cap) overflow = true;
-            if (!overflow && hi > lo)
-                FG_CUDA(c, cudaMemcpyAsync(c->h_enc_out + lo, c->d_enc_out + lo, (size_t)(hi - lo), cudaMemcpyDeviceToHost, c->s_d2h));
-        }
-        uint32_t total[kCnt];
-        memcpy(total, c->h_counts + (size_t)(chunks - 1) * kCnt, sizeof total);
-        FG_CUDA(c, cudaStreamSynchronize(c->s_d2h));
-        if (total[kBadFlag]) return fail(c, FG_E_ARG, "offsets must be non-decreasing and within max_batch_bytes");
-        if (overflow) {
-            if (tables_overflow(c, (int)fmt, total))
-                if (int rc = regrow_tables(c, (int)fmt, total)) return rc;
-            const unsigned long long need = c->h_enc_base[chunks];
-            if (need > c->enc_out_cap)
-                if (int rc = alloc_enc_out(c, (size_t)need + (size_t)need / 8 + 4096)) return rc;
-            out->bytes = c->h_enc_out;
+        uint32_t total[fg::K5_COUNT];
+        float kms = 0.f;
+        const int rc = drain(c, fmt, chunks, copy_records, total, &kms);
+        if (rc == kRedo) {
+            const unsigned long long need = base[chunks];
+            if (need > c->enc_out.cap) FG_CUDA(c, c->enc_out.alloc((size_t)need + (size_t)need / 8 + 4096));
+            out->bytes = c->enc_out.h;
             continue;
         }
-        float kms = 0.f;
-        for (int k = 0; k < chunks; ++k) {
-            float ms = 0.f;
-            FG_CUDA(c, cudaEventElapsedTime(&ms, c->ev_k0[k], c->ev_k1[k]));
-            kms += ms;
-        }
+        if (rc) return rc;
         out->n = n;
         out->kernel_ms = kms;
         out->total_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t_begin).count();
@@ -1216,7 +1138,6 @@ int fg_split_decode_framed(fg_ctx* c, fg_format fmt, fg_framing framing, const u
         FG_CUDA(c, cudaMalloc(&c->d_seg, sizeof(uint32_t) * ((size_t)fg::split_segments((long long)c->max_bytes) + 16)));
         FG_CUDA(c, cudaMalloc(&c->d_n_lines, 256));
         FG_CUDA(c, cudaMalloc(&c->d_invalid, (size_t)c->max_lines + 64));
-        FG_CUDA(c, cudaHostAlloc(&c->h_offsets, sizeof(int32_t) * ((size_t)c->max_lines + 1), cudaHostAllocDefault));
         FG_CUDA(c, cudaHostAlloc(&c->h_n_lines, 64, cudaHostAllocDefault));
         FG_CUDA(c, cudaEventCreate(&c->ev_s0));
         FG_CUDA(c, cudaEventCreate(&c->ev_s1));
@@ -1229,20 +1150,19 @@ int fg_split_decode_framed(fg_ctx* c, fg_format fmt, fg_framing framing, const u
             FG_CUDA(c, cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
             c->ev_split.push_back(e);
         }
-        dfree(c->d_cum);
-        hfree(c->h_cum);
-        FG_CUDA(c, cudaMalloc(&c->d_cum, sizeof(int32_t) * want));
-        FG_CUDA(c, cudaHostAlloc(&c->h_cum, sizeof(int32_t) * want, cudaHostAllocDefault));
+        FG_CUDA(c, c->cum.alloc(want));
     }
     if (int rc = ensure_events(c, chunks + 1)) return rc;
     memset(out, 0, sizeof *out);
     const bool pinned = nbytes > 0 && is_pinned(stream);
+    const int32_t* cum = c->cum.host<int32_t>();
+    auto copy_tables = [&](int, const uint32_t* prev, const uint32_t* cur) { return copy_tables_d2h(c, fmt, prev, cur); };
 
     for (int attempt = 0; attempt < 2; ++attempt) {
         // ---- enqueue, chunk by chunk: raw bytes -> HBM, then framing + UTF-8 validation of that chunk (no host dependency)
         FG_CUDA(c, cudaMemsetAsync(c->d_n_lines + 8, 0, 4, c->s_comp));  // running newline count (uint32 at d_n_lines[8])
         FG_CUDA(c, cudaMemsetAsync(c->d_invalid, 0, (size_t)c->max_lines, c->s_comp));
-        FG_CUDA(c, cudaMemsetAsync(c->d_k, 0, sizeof(uint32_t) * kCnt, c->s_comp));
+        FG_CUDA(c, cudaMemsetAsync(c->d_k, 0, sizeof(uint32_t) * fg::K5_COUNT, c->s_comp));
         FG_CUDA(c, cudaEventRecord(c->ev_s0, c->s_comp));
         int bounce_ix = 0;
         for (int k = 0; k < chunks; ++k) {
@@ -1253,9 +1173,10 @@ int fg_split_decode_framed(fg_ctx* c, fg_format fmt, fg_framing framing, const u
             FG_CUDA(c, cudaEventRecord(c->ev_h2d[k], c->s_h2d));
             FG_CUDA(c, cudaStreamWaitEvent(c->s_comp, c->ev_h2d[k], 0));
             FG_CUDA(c, fg::launch_split_chunk(c->d_bytes, (long long)nbytes, c0, c1, last ? 1 : 0, c->d_seg, (uint32_t*)(c->d_n_lines + 8),
-                                              c->d_cum + k, c->d_offsets, c->d_n_lines, c->max_lines, c->d_invalid, delim, c->s_comp));
+                                              c->cum.dev<int32_t>() + k, c->offsets.dev<int32_t>(), c->d_n_lines, c->max_lines,
+                                              c->d_invalid, delim, c->s_comp));
             c->launches += 4;
-            FG_CUDA(c, cudaMemcpyAsync(c->h_cum + k, c->d_cum + k, 4, cudaMemcpyDeviceToHost, c->s_comp));
+            FG_CUDA(c, c->cum.d2h(k, k + 1, c->s_comp));
             if (last) {
                 FG_CUDA(c, cudaMemcpyAsync(c->h_n_lines, c->d_n_lines, 4, cudaMemcpyDeviceToHost, c->s_comp));
                 FG_CUDA(c, cudaEventRecord(c->ev_s1, c->s_comp));
@@ -1271,7 +1192,7 @@ int fg_split_decode_framed(fg_ctx* c, fg_format fmt, fg_framing framing, const u
         for (int k = 0; k < chunks; ++k) {
             const int dep = std::min(k + 1, chunks - 1);
             FG_CUDA(c, cudaEventSynchronize(c->ev_split[dep]));
-            int32_t upto = c->h_cum[k];
+            int32_t upto = cum[k];
             if (upto < 0) { over = true; break; }
             if (k == chunks - 1) {
                 n = *c->h_n_lines;
@@ -1285,10 +1206,7 @@ int fg_split_decode_framed(fg_ctx* c, fg_format fmt, fg_framing framing, const u
                 FG_CUDA(c, cudaStreamWaitEvent(c->s_parse, c->ev_split[dep], 0));
                 FG_CUDA(c, cudaEventRecord(c->ev_k0[nparse], c->s_parse));
                 if (int rc = launch_lines(c, (int)fmt, done_lines, cnt, tile, c->d_invalid + done_lines, strip, c->s_parse)) return rc;
-                FG_CUDA(c, cudaEventRecord(c->ev_k1[nparse], c->s_parse));
-                FG_CUDA(c, cudaMemcpyAsync(c->h_counts + (size_t)nparse * kCnt, c->d_k, sizeof(uint32_t) * kCnt, cudaMemcpyDeviceToHost, c->s_parse));
-                FG_CUDA(c, cudaEventRecord(c->ev_cnt[nparse], c->s_parse));
-                FG_CUDA(c, cudaStreamWaitEvent(c->s_d2h, c->ev_cnt[nparse], 0));
+                if (int rc = end_step(c, nparse, c->s_parse)) return rc;
                 if (int rc = copy_rows_d2h(c, fmt, done_lines, cnt, c->s_d2h)) return rc;
                 ++nparse;
                 done_lines = upto;
@@ -1299,35 +1217,17 @@ int fg_split_decode_framed(fg_ctx* c, fg_format fmt, fg_framing framing, const u
             return fail(c, FG_E_CAPACITY, "stream has more lines than max_batch_lines");
         }
         // ---- side table ranges, line offsets
-        uint32_t prev[kCnt] = {}, total[kCnt] = {};
-        bool overflow = false;
-        for (int j = 0; j < nparse; ++j) {
-            FG_CUDA(c, cudaEventSynchronize(c->ev_cnt[j]));
-            const uint32_t* cur = c->h_counts + (size_t)j * kCnt;
-            memcpy(total, cur, sizeof total);
-            if (tables_overflow(c, (int)fmt, cur)) { overflow = true; continue; }
-            if (!overflow) {
-                if (int rc = copy_tables_d2h(c, (int)fmt, prev, cur, c->s_d2h)) return rc;
-                memcpy(prev, cur, sizeof prev);
-            }
-        }
-        if (overflow) {
-            FG_CUDA(c, cudaDeviceSynchronize());
-            if (int rc = regrow_tables(c, (int)fmt, total)) return rc;
-            continue;
-        }
-        FG_CUDA(c, cudaStreamSynchronize(c->s_parse));
-        FG_CUDA(c, cudaMemcpyAsync(c->h_offsets, c->d_offsets, sizeof(int32_t) * ((size_t)n + 1), cudaMemcpyDeviceToHost, c->s_d2h));
-        FG_CUDA(c, cudaStreamSynchronize(c->s_d2h));
+        uint32_t total[fg::K5_COUNT];
         float kms = 0.f;
-        for (int j = 0; j < nparse; ++j) {
-            float ms = 0.f;
-            FG_CUDA(c, cudaEventElapsedTime(&ms, c->ev_k0[j], c->ev_k1[j]));
-            kms += ms;
-        }
+        const int rc = drain(c, fmt, nparse, copy_tables, total, &kms);
+        if (rc == kRedo) continue;
+        if (rc) return rc;
+        FG_CUDA(c, cudaStreamSynchronize(c->s_parse));
+        FG_CUDA(c, c->offsets.d2h(0, (size_t)n + 1, c->s_d2h));
+        FG_CUDA(c, cudaStreamSynchronize(c->s_d2h));
         FG_CUDA(c, cudaEventElapsedTime(&c->last_split_ms, c->ev_s0, c->ev_s1));  // includes waiting for the H2D chunks
         fill_out(c, fmt, n, total, out);
-        out->line_offsets = c->h_offsets;
+        out->line_offsets = c->offsets.host<int32_t>();
         out->kernel_ms = kms;
         out->total_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t_begin).count();
         return FG_OK;
@@ -1341,17 +1241,17 @@ int fg_upload(fg_ctx* c, const uint8_t* bytes, const int32_t* offsets, int32_t n
     if (n > 0) {
         const size_t b0 = (size_t)offsets[0], b1 = (size_t)offsets[n];
         FG_CUDA(c, cudaMemcpy(c->d_bytes + b0, bytes + b0, b1 - b0, cudaMemcpyHostToDevice));
-        FG_CUDA(c, cudaMemcpy(c->d_offsets, offsets, sizeof(int32_t) * ((size_t)n + 1), cudaMemcpyHostToDevice));
+        FG_CUDA(c, cudaMemcpy(c->offsets.d, offsets, sizeof(int32_t) * ((size_t)n + 1), cudaMemcpyHostToDevice));
         c->res_bytes = b1 - b0;
     } else {
         c->res_bytes = 0;
     }
-    FG_CUDA(c, cudaMemset(c->d_k, 0, sizeof(uint32_t) * kCnt));
-    FG_CUDA(c, fg::launch_check_offsets(c->d_offsets, n, (long long)c->max_bytes, c->d_k + kBadFlag, c->s_comp));
+    FG_CUDA(c, cudaMemset(c->d_k, 0, sizeof(uint32_t) * fg::K5_COUNT));
+    FG_CUDA(c, fg::launch_check_offsets(c->offsets.dev<int32_t>(), n, (long long)c->max_bytes, c->d_k + fg::K5_BAD_OFFSETS, c->s_comp));
     uint32_t bad = 0;
-    FG_CUDA(c, cudaMemcpyAsync(&bad, c->d_k + kBadFlag, 4, cudaMemcpyDeviceToHost, c->s_comp));
+    FG_CUDA(c, cudaMemcpyAsync(&bad, c->d_k + fg::K5_BAD_OFFSETS, 4, cudaMemcpyDeviceToHost, c->s_comp));
     FG_CUDA(c, cudaStreamSynchronize(c->s_comp));
-    if (bad) return fail(c, FG_E_ARG, "offsets must be non-decreasing and within max_batch_bytes");
+    if (bad) return fail(c, FG_E_ARG, kBadOffsets);
     c->res_n = n;
     c->res_fmt = -1;
     return FG_OK;
@@ -1364,11 +1264,11 @@ int fg_parse_resident(fg_ctx* c, fg_format fmt, float* kernel_ms) {
     if (int rc = ensure_format(c, (int)fmt)) return rc;
     c->call_year = current_year(c);
     for (int attempt = 0; attempt < 2; ++attempt) {
-        FG_CUDA(c, cudaMemsetAsync(c->d_k, 0, sizeof(uint32_t) * kBadFlag, c->s_comp));
+        FG_CUDA(c, cudaMemsetAsync(c->d_k, 0, sizeof(uint32_t) * fg::K5_BAD_OFFSETS, c->s_comp));
         FG_CUDA(c, cudaEventRecord(c->ev_a, c->s_comp));
         if (int rc = launch_lines(c, (int)fmt, 0, c->res_n, pick_tile(c, c->res_bytes, c->res_n, (int)fmt), nullptr, 0, c->s_comp, true)) return rc;
         FG_CUDA(c, cudaEventRecord(c->ev_b, c->s_comp));
-        uint32_t total[kCnt] = {};
+        uint32_t total[fg::K5_COUNT] = {};
         FG_CUDA(c, cudaMemcpyAsync(total, c->d_k, sizeof total, cudaMemcpyDeviceToHost, c->s_comp));
         FG_CUDA(c, cudaStreamSynchronize(c->s_comp));
         if (tables_overflow(c, (int)fmt, total)) {
@@ -1398,11 +1298,11 @@ int fg_parse_resident_n(fg_ctx* c, fg_format fmt, int32_t k, float* total_ms) {
     const int tile = pick_tile(c, c->res_bytes, c->res_n, (int)fmt);
     FG_CUDA(c, cudaEventRecord(c->ev_a, c->s_comp));
     for (int32_t it = 0; it < k; ++it) {
-        FG_CUDA(c, cudaMemsetAsync(c->d_k, 0, sizeof(uint32_t) * kBadFlag, c->s_comp));
+        FG_CUDA(c, cudaMemsetAsync(c->d_k, 0, sizeof(uint32_t) * fg::K5_BAD_OFFSETS, c->s_comp));
         if (int rc = launch_lines(c, (int)fmt, 0, c->res_n, tile, nullptr, 0, c->s_comp)) return rc;
     }
     FG_CUDA(c, cudaEventRecord(c->ev_b, c->s_comp));
-    uint32_t total[kCnt] = {};
+    uint32_t total[fg::K5_COUNT] = {};
     FG_CUDA(c, cudaMemcpyAsync(total, c->d_k, sizeof total, cudaMemcpyDeviceToHost, c->s_comp));
     FG_CUDA(c, cudaStreamSynchronize(c->s_comp));
     if (tables_overflow(c, (int)fmt, total))
@@ -1420,9 +1320,9 @@ int fg_download(fg_ctx* c, fg_format fmt, fg_batch_out* out) {
     if (c->res_fmt != (int)fmt) return fail(c, FG_E_ARG, "no resident parse of this format to download");
     FG_CUDA(c, cudaSetDevice(c->device));
     memset(out, 0, sizeof *out);
-    const uint32_t zero[kCnt] = {};
+    const uint32_t zero[fg::K5_COUNT] = {};
     if (int rc = copy_rows_d2h(c, fmt, 0, c->res_n, c->s_d2h)) return rc;
-    if (int rc = copy_tables_d2h(c, (int)fmt, zero, c->res_tot, c->s_d2h)) return rc;
+    if (int rc = copy_tables_d2h(c, fmt, zero, c->res_tot)) return rc;
     FG_CUDA(c, cudaStreamSynchronize(c->s_d2h));
     fill_out(c, fmt, c->res_n, c->res_tot, out);
     return FG_OK;

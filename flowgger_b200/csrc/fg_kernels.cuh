@@ -102,7 +102,7 @@ struct WideRow {
 };
 static_assert(sizeof(WideRow) == 72, "WideRow must be 72 bytes");
 
-enum { K5_ENTRIES = 0, K5_ARENA = 1, K5_WIDE_ROWS = 2, K5_WIDE_ENTRIES = 3, K5_ESC_LIST = 4, K5_WIDE_LIST = 5, K5_COUNT = 8 };
+enum { K5_ENTRIES = 0, K5_ARENA = 1, K5_WIDE_ROWS = 2, K5_WIDE_ENTRIES = 3, K5_ESC_LIST = 4, K5_WIDE_LIST = 5, K5_BAD_OFFSETS = 6, K5_COUNT = 8 };
 
 struct Parse5424Params {
     const uint8_t* bytes;
